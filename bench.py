@@ -3,6 +3,7 @@
 
   python bench.py [--gpus N] [--steps K] [--warmup W]            our CUDA path (one process per GPU under torchrun)
   python bench.py --impl reference [...]                         the reference's own CPU estimateGround on the host cores
+  python bench.py [...] --dump-outputs DIR                       also write what the last timed step computed to DIR/*.npy
 
 Workload (BASELINE.json configs[2], the configuration the metric is quoted on): a batch of 1024 synthetic KITTI-64
 frames (~120k points each) per GPU, each frame on its own FRESH stream state. A "step" is one pass of the whole path
@@ -31,7 +32,7 @@ import time
 
 REPO = os.path.dirname(os.path.abspath(__file__))
 PKG = os.path.join(REPO, "patchwork-plusplus_b200")
-for p in (PKG, os.path.join(PKG, "lib")):
+for p in (PKG, os.path.join(PKG, "lib"), os.path.join(REPO, "tests")):
     if p not in sys.path:
         sys.path.insert(0, p)
 
@@ -39,6 +40,8 @@ SEED = 20260922
 METRIC = "frames/sec (120k-pt KITTI cloud)"
 UNIT = "frames/s"
 ALGO_BYTES_PER_POINT = 20  # SURVEY.md §8(d): 16 B/pt compulsory read of the N x 4 f32 cloud + 4 B/pt int32 index write
+DUMP_SAMPLE_FRAMES = 32          # --dump-outputs: index lists of at most this many frames,
+DUMP_LIST_BYTES = 48 << 20       # and at most this many bytes of them (everything dumped stays under 64 MB)
 
 
 def parse():
@@ -57,7 +60,14 @@ def parse():
     ap.add_argument("--streaming", default="64x16", help="streaming mode 'SxT': S sensor streams x T consecutive frames each, T batched calls with the temporal state carried (SURVEY.md 8d config 3); reported under the key 'streaming' ('' = skip)")
     ap.add_argument("--no-extras", action="store_true", help="skip the extra records: streaming, dense1m (BASELINE config 5 shape, 32 frames per GPU), latency_us (config 2), parity_vs_reference")
     ap.add_argument("--dense-frames", type=int, default=32, help="frames per GPU of the dense1m sub-record")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed to DIR/<name>.npy "
+                    "(float64 / float32): per-frame counts, heights and a fixed, seeded sample of frames' index lists, centers and normals")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl ours)")
+    return a
 
 
 def merge_front_stages(stage_ms):
@@ -232,6 +242,33 @@ def cpu_reference_throughput(frames, seconds_budget, max_frames=None, threads=No
             "sample": f"{n} estimateGround calls over {min(lim, len(frames))} frames of the same synthetic batch, fresh instance per call, {dt:.1f} s wall on {T} threads"}, n, dt
 
 
+def dump_outputs(eng, nframes, out_dir):
+    """What the engine's last call computed, read back through the C-ABI like a caller would: per frame the ground / non-ground
+    counts, the number of patches and the sensor height; for a sample of frames drawn with the bench seed (the same frames from
+    run to run) their ground and non-ground index lists in emission order, concatenated in ascending frame order, and the patch
+    centers and normals. Integers are written as float64 (exact), the engine's float32 outputs as float32."""
+    import numpy as np
+    counts = {name: np.array([fn(f) for f in range(nframes)], np.float64) for name, fn in
+              (("num_ground", eng.num_ground), ("num_nonground", eng.num_nonground), ("num_patches", eng.num_patches), ("height", eng.height))}
+    sample, list_bytes = [], 0
+    for f in np.random.default_rng(SEED).permutation(nframes)[:DUMP_SAMPLE_FRAMES]:
+        nb = 8 * int(counts["num_ground"][f] + counts["num_nonground"][f])
+        if sample and list_bytes + nb > DUMP_LIST_BYTES:
+            break
+        sample.append(int(f))
+        list_bytes += nb
+    sample.sort()
+    out = dict(counts, sample_frames=np.array(sample, np.float64))
+    for name, fn, dtype in (("ground_indices", eng.ground_indices, np.float64), ("nonground_indices", eng.nonground_indices, np.float64),
+                            ("centers", eng.centers, np.float32), ("normals", eng.normals, np.float32)):
+        out[name] = np.concatenate([fn(f) for f in sample]).astype(dtype)
+    total = sum(a.nbytes for a in out.values())
+    assert total <= 64 << 20, f"--dump-outputs: {total} bytes"
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 # ----------------------------------------------------------------------------------------------------------------
 def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
@@ -338,6 +375,8 @@ def run_ours(args):
         clk = clk_nvml
     ms = ev0.elapsed_time(ev1)
     launches = eng.launch_count() - launches0
+    if args.dump_outputs:
+        dump_outputs(eng, F, args.dump_outputs if world == 1 else os.path.join(args.dump_outputs, f"rank{rank}"))
     # per-kernel device times: the same steps once more with CUDA events around every kernel (the five fit kernels,
     # which otherwise overlap on side streams, are serialised for this)
     eng.set_profiling(True)
@@ -529,33 +568,29 @@ def run_ours(args):
     real, rms = None, -1.0
     if not args.no_extras and args.sensor == "kitti64":
         try:
-            scans = []
-            for i in range(6):
-                gp = os.path.join(REPO, "tests", "golden", f"kitti_{i:06d}.npz")
-                if os.path.exists(gp):
-                    scans.append(torch.from_numpy(np.ascontiguousarray(np.load(gp)["xyzi_t"].T)))
-            if scans:
-                sizes = [int(scans[f % len(scans)].shape[0]) for f in range(F)]
-                roffs_np = np.zeros(F + 1, np.int64); roffs_np[1:] = np.cumsum(sizes)
-                dscans = [x.to(dev) for x in scans]
-                rpts = torch.cat([dscans[f % len(scans)] for f in range(F)], dim=0).contiguous()
-                reng = pwpp_b200.Engine(device=local, num_streams=F, max_points_per_frame=max(sizes))
+            from conftest import load_kitti
+            scans = [torch.from_numpy(load_kitti(i)) for i in range(6)]
+            sizes = [int(scans[f % len(scans)].shape[0]) for f in range(F)]
+            roffs_np = np.zeros(F + 1, np.int64); roffs_np[1:] = np.cumsum(sizes)
+            dscans = [x.to(dev) for x in scans]
+            rpts = torch.cat([dscans[f % len(scans)] for f in range(F)], dim=0).contiguous()
+            reng = pwpp_b200.Engine(device=local, num_streams=F, max_points_per_frame=max(sizes))
 
-                def rstep():
-                    reng.reset(); reng.estimate_device(rpts.data_ptr(), roffs_np, True, stream)
-                for _ in range(3):
-                    rstep()
-                torch.cuda.synchronize()
-                r0, r1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-                r0.record()
-                for _ in range(5):
-                    rstep()
-                r1.record(); torch.cuda.synchronize()
-                rms = r0.elapsed_time(r1) / 5
-                reng.set_profiling(True); rstep(); rstage = merge_front_stages(reng.stage_times_ms()); reng.set_profiling(False)
-                assert reng.num_ground(7) + reng.num_nonground(7) == sizes[7]
-                rground = float(np.mean([reng.num_ground(f) / sizes[f] for f in range(6)]))
-                reng.close(); del rpts, dscans
+            def rstep():
+                reng.reset(); reng.estimate_device(rpts.data_ptr(), roffs_np, True, stream)
+            for _ in range(3):
+                rstep()
+            torch.cuda.synchronize()
+            r0, r1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            r0.record()
+            for _ in range(5):
+                rstep()
+            r1.record(); torch.cuda.synchronize()
+            rms = r0.elapsed_time(r1) / 5
+            reng.set_profiling(True); rstep(); rstage = merge_front_stages(reng.stage_times_ms()); reng.set_profiling(False)
+            assert reng.num_ground(7) + reng.num_nonground(7) == sizes[7]
+            rground = float(np.mean([reng.num_ground(f) / sizes[f] for f in range(6)]))
+            reng.close(); del rpts, dscans
         except Exception as ex:
             real = {"error": repr(ex)[:200]}
         rms = dist.max_over_ranks(rms)
@@ -569,10 +604,10 @@ def run_ours(args):
     if rank == 0 and not args.no_extras:
         try:
             exe = os.path.join(PKG, "lib", "pwpp_latency")
-            gold = os.path.join(REPO, "tests", "golden", "kitti_000000.npz")
-            if os.path.exists(exe) and os.path.exists(gold):
+            if os.path.exists(exe):
                 import tempfile
-                scan = np.ascontiguousarray(np.load(gold)["xyzi_t"].T)
+                from conftest import load_kitti
+                scan = load_kitti(0)
                 with tempfile.NamedTemporaryFile(suffix=".bin") as tf:
                     scan.tofile(tf.name)
                     env = dict(os.environ, CUDA_VISIBLE_DEVICES=str(local))

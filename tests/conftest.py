@@ -68,9 +68,9 @@ def build_simt(force=False):
 
 
 def load_kitti(f: int) -> np.ndarray:
-    """The reference's fixture scan data/00000f.bin (N x 4 float32), from the committed copy."""
-    z = np.load(os.path.join(HERE, "golden", f"kitti_{f:06d}.npz"))
-    return np.ascontiguousarray(z["xyzi_t"].T)
+    """The reference's fixture scan data/00000f.bin (N x 4 float32), from the committed copy (two halves of the points)."""
+    halves = [np.load(os.path.join(HERE, "golden", f"kitti_{f:06d}_{h}.npz"))["xyzi_t"] for h in "ab"]
+    return np.ascontiguousarray(np.concatenate(halves, axis=1).T)
 
 
 @pytest.fixture(scope="session")
@@ -81,3 +81,9 @@ def kitti():
 @pytest.fixture(scope="session")
 def golden():
     return np.load(os.path.join(HERE, "golden", "golden_ref.npz"))
+
+
+@pytest.fixture(scope="session")
+def refout():
+    from helpers import ReferenceOutputs
+    return ReferenceOutputs(os.path.join(HERE, "golden", "reference_outputs.npz"))

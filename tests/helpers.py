@@ -1,5 +1,6 @@
 """Shared comparison helpers for the parity tests."""
 import ctypes as C
+import hashlib
 import os
 
 import numpy as np
@@ -42,25 +43,103 @@ class Twin(_Base):
         return self._lib.twin_fast_mismatches(self._h)
 
 
-def bits(a):
+# Everything the reference surface exposes after an estimate (including emission order), the adaptive state and its
+# histories; then the label SETS (the index lists sorted).
+SURFACE = ("getGroundIndices", "getNongroundIndices", "getGround", "getNonground", "getCenters", "getNormals", "state",
+           "history_sizes") + tuple(f"history_{r}_{w}" for r in range(4) for w in (0, 1))
+SETS = ("ground_set", "nonground_set")
+
+
+def surface_array(obj, name):
+    """One entry of SURFACE + SETS of an oracle / reference / twin object that has just estimated a frame."""
+    if name.startswith("get"):
+        return getattr(obj, name)()
+    if name in SETS:
+        return np.sort(obj.getGroundIndices() if name == "ground_set" else obj.getNongroundIndices())
+    st = obj.state()
+    if name == "state":
+        return np.array([st.sensor_height, *st.elevation_thr, *st.flatness_thr], dtype=np.float64)
+    if name == "history_sizes":
+        return np.array([*st.n_elevation, *st.n_flatness], dtype=np.int32)
+    _, r, w = name.split("_")
+    return obj.history(int(r), int(w))
+
+
+def digest(a) -> np.ndarray:
+    """16-byte BLAKE2b of an array's dtype, shape and bytes: equal digests mean bit-identical arrays."""
     a = np.ascontiguousarray(a)
-    return a.view(np.uint32) if a.dtype == np.float32 else (a.view(np.uint64) if a.dtype == np.float64 else a)
+    h = hashlib.blake2b(f"{a.dtype.str}{a.shape}".encode(), digest_size=16)
+    h.update(a.tobytes())
+    return np.frombuffer(h.digest(), dtype=np.uint8)
 
 
-def assert_bit_identical(a, b, what=""):
-    """Everything the reference surface exposes, bit for bit, including emission order."""
-    for name in ("getGroundIndices", "getNongroundIndices", "getGround", "getNonground", "getCenters", "getNormals"):
-        x, y = getattr(a, name)(), getattr(b, name)()
-        assert x.shape == y.shape, f"{what} {name}: shape {x.shape} vs {y.shape}"
-        assert np.array_equal(bits(x), bits(y)), f"{what} {name}: values differ"
-    sa, sb = a.state(), b.state()
-    assert bits(np.float64(sa.sensor_height)) == bits(np.float64(sb.sensor_height)), f"{what} sensor_height"
-    for fld in ("elevation_thr", "flatness_thr"):
-        assert np.array_equal(bits(np.array(getattr(sa, fld))), bits(np.array(getattr(sb, fld)))), f"{what} {fld}"
-    assert list(sa.n_elevation) == list(sb.n_elevation) and list(sa.n_flatness) == list(sb.n_flatness), f"{what} history sizes"
-    for r in range(4):
-        for w in (0, 1):
-            assert np.array_equal(bits(a.history(r, w)), bits(b.history(r, w))), f"{what} history ring {r} kind {w}"
+class ReferenceOutputs:
+    """tests/golden/reference_outputs.npz, written by tests/golden/make_golden.py: what the reference's own estimateGround
+    returned on the inputs of the tests that compare with it. Per case: digests of the input and of every SURFACE + SETS
+    array; for the synthetic batches also the ground mask of every frame, so that differing labels can be counted."""
+
+    def __init__(self, path):
+        z = np.load(path)
+        self._digests = dict(zip(z["digest_keys"].tolist(), z["digests"]))
+        self._arrays = {k: z[k] for k in z.files if k not in ("digest_keys", "digests")}
+
+    def digest(self, case, name):
+        return self._digests[f"{case}|{name}"]
+
+    def check_input(self, case, a):
+        assert np.array_equal(digest(np.ascontiguousarray(a, dtype=np.float32)), self.digest(case, "input")), \
+            f"{case}: not the input the reference outputs were recorded on"
+
+    def assert_matches(self, case, a, obj, names=SURFACE):
+        """obj, which has just estimated `a`, returns bit for bit what the reference returned on this case."""
+        self.check_input(case, a)
+        for name in names:
+            assert np.array_equal(digest(surface_array(obj, name)), self.digest(case, name)), f"{case}: {name} differs from the reference"
+
+    def ground_masks(self, batch):
+        """The reference's ground mask of every frame of a recorded batch, and the number of points it emitted per frame."""
+        n = self._arrays[batch + "/n"]
+        bits = np.unpackbits(self._arrays[batch + "/ground_mask"])[:n.sum()].astype(bool)
+        return np.split(bits, np.cumsum(n)[:-1]), self._arrays[batch + "/emitted"]
+
+
+# Inputs built by hand for the comparisons with the reference (also used by tests/golden/make_golden.py).
+def edge_inputs():
+    rng = np.random.default_rng(7)
+    return {
+        "empty": np.zeros((0, 4), np.float32),
+        "one_point": np.array([[5, 0, -1.7, 0.5]], np.float32),
+        "nine_in_one_bin": np.c_[5 + rng.random(9) * 0.1, rng.random(9) * 0.1, -1.7 + rng.random(9) * 0.01, rng.random(9)].astype(np.float32),
+        "all_out_of_range": np.c_[rng.random((50, 2)) * 1.0, rng.random((50, 2))].astype(np.float32),
+        "flat_plane": np.c_[(rng.random((5000, 2)) - 0.5) * 60, np.full(5000, -1.723), rng.random(5000)].astype(np.float32),
+        "axis_points": np.array([[10, 0, -1.7, .5], [-10, 0, -1.7, .5], [0, 10, -1.7, .5], [0, -10, -1.7, .5], [3, -0.0, -1.7, .5]] * 4, np.float32),
+    }
+
+
+def wall_frame():
+    """A wall inside a zone-0 bin: R-VPF removes points in several iterations."""
+    rng = np.random.default_rng(11)
+    return np.r_[np.c_[4 + rng.random(6000) * 0.05, rng.random(6000) * 0.6, -1.7 + rng.random(6000) * 2.0, rng.random(6000)],
+                 np.c_[3 + rng.random(6000) * 4, rng.random(6000) * 0.6, -1.7 + rng.normal(0, 0.02, 6000), rng.random(6000)]].astype(np.float32)
+
+
+def ties_frame():
+    """A synthetic scan with centimetre-quantised z: thousands of exact ties per bin."""
+    import synth
+    b = synth.make_frame(20260922, 1).numpy()
+    b[:, 2] = np.round(b[:, 2] / 0.01) * 0.01
+    return b
+
+
+FLAT_PATCH_SIZES = [10, 15, 16, 17, 31, 33, 63, 64, 65, 127, 129, 255, 256, 257, 511, 512, 513, 1023, 1025, 2047, 2048, 2049, 4095,
+                    4096, 4097, 8191, 8192]
+
+
+def flat_patch_frames():
+    """One flat patch per frame, of each of FLAT_PATCH_SIZES points."""
+    rng = np.random.default_rng(5)
+    return [np.c_[5 + rng.random(n) * 0.5, rng.random(n) * 0.5, -1.7 + rng.normal(0, 0.03, n), rng.random(n)].astype(np.float32)
+            for n in FLAT_PATCH_SIZES]
 
 
 # stated floating-point tolerances of the CANON64 contract (DESIGN.md §3)

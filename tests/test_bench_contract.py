@@ -62,3 +62,38 @@ def test_front_end_stage_slots_are_merged_only_for_the_cluster_kernel():
         r = j["roofline"]
         assert r["bound"] == "hbm" and abs(r["frac"] - r["achieved"] / r["peak"]) < 1e-9 and r["traffic"] is not None and "k_front" in r["per_kernel"]
         assert j["e2e"]["h2d_bytes_per_step"] > 0 and j["e2e"]["d2h_bytes_per_step"] > 0 and j["gpu_launches"] > 0
+
+
+def test_dump_outputs_writes_the_same_seeded_sample(tmp_path):
+    """--dump-outputs: per-frame records of every frame, and the index lists, centers and normals of a sample of frames that is
+    the same from run to run, in float64 / float32 only."""
+    import numpy as np
+    sys.path.insert(0, REPO)
+    import importlib
+    bench = importlib.import_module("bench")
+
+    class Engine:   # the getters of pwpp_b200.Engine that dump_outputs reads; frame f: f + 1 ground points, 2 non-ground, one patch
+        num_ground = staticmethod(lambda f: f + 1)
+        num_nonground = staticmethod(lambda f: 2)
+        num_patches = staticmethod(lambda f: 1)
+        height = staticmethod(lambda f: 1.5 + f)
+        ground_indices = staticmethod(lambda f: np.arange(f + 1, dtype=np.int32))
+        nonground_indices = staticmethod(lambda f: np.array([f + 1, f + 2], np.int32))
+        centers = staticmethod(lambda f: np.full((1, 3), f, np.float32))
+        normals = staticmethod(lambda f: np.full((1, 3), -f, np.float32))
+
+    for d in ("a", "b"):
+        bench.dump_outputs(Engine(), 100, str(tmp_path / d))
+    names = sorted(os.listdir(tmp_path / "a"))
+    assert names == sorted(os.listdir(tmp_path / "b")) and "ground_indices.npy" in names and "num_ground.npy" in names
+    out = {}
+    for n in names:
+        a, b = np.load(tmp_path / "a" / n), np.load(tmp_path / "b" / n)
+        assert a.dtype in (np.float32, np.float64) and a.dtype == b.dtype and np.array_equal(a, b), n
+        out[n[:-4]] = a
+    sample = out["sample_frames"].astype(int)
+    assert len(sample) == bench.DUMP_SAMPLE_FRAMES and np.all(np.diff(sample) > 0)
+    assert np.array_equal(out["num_ground"], np.arange(1, 101)) and np.array_equal(out["height"], 1.5 + np.arange(100))
+    assert np.array_equal(out["ground_indices"], np.concatenate([np.arange(f + 1) for f in sample]))
+    assert np.array_equal(out["nonground_indices"], np.concatenate([[f + 1, f + 2] for f in sample]))
+    assert np.array_equal(out["centers"][:, 0], sample) and out["normals"].shape == (len(sample), 3)

@@ -2,8 +2,9 @@
 
   * the committed golden vectors of all three parameter sets (tests/golden/golden_ref.npz, produced by the reference's
     own patchworkpp.cpp, tests/golden/make_golden.py), fresh and sequential;
-  * oracle/_ref/libpwref.so (the reference's sources compiled where they lie; the built .so travels to the GPU box) run
-    side by side on >= 256 frames of the benchmark's synthetic config-3 batch and on a dense config-5-shaped frame;
+  * what the reference build (oracle/_ref/libpwref.so, the reference's sources compiled against oracle/eigen_shim) returned on
+    256 frames of the benchmark's synthetic config-3 batch and on a dense config-5-shaped frame, and the index lists of its
+    stable-sort variant, recorded in tests/golden/reference_outputs.npz (tests/golden/make_golden.py);
   * the same on a second device when the box has more than one GPU (BASELINE config 4: no parity claim without it).
 
 The reference computes in fp32, the CUDA path in double (DESIGN.md §3): labels are compared exactly and the number of
@@ -11,12 +12,11 @@ differing labels is reported and bounded — on data with points within fp32 rou
 legitimately disagree on that point (measured: 1 label in 1.4 M on the synthetic scans); patches whose plane was fitted to
 fewer than 3 points are numerically undefined in the reference too and are excluded (oracle.bin_min_fit_n).
 """
-import os
-
 import numpy as np
 import pytest
 
 import oracle_py as O
+from helpers import digest, wall_frame
 from param_sets import PARAM_SETS
 
 pytestmark = pytest.mark.gpu
@@ -75,18 +75,15 @@ def test_golden_sequence_no_rvpf_tgr(kitti, golden):
         assert np.array_equal(m, gm), f"seq frame {f}: {int((m != gm).sum())} labels differ from the reference golden"
 
 
-def _compare_with_reference(eng, frames, what):
-    """labels of the engine's frames vs libpwref.so run on the same arrays; returns (labels, mismatches)."""
+def _compare_with_reference(eng, frames, refout, batch):
+    """labels of the engine's frames vs the reference's labels recorded on the same arrays; returns (labels, mismatches)."""
+    masks, emitted = refout.ground_masks(batch)
     labels = mism = 0
     for f, a in enumerate(frames):
-        ref = O.Reference(stable_sort=False)
-        ref.estimate(a)
-        g_r = ref.getGroundIndices()
-        n_r = ref.getNongroundIndices()
-        ref.close()
+        refout.check_input(f"{batch}/{f}", a)
         g_e, n_e = eng.ground_indices(f), eng.nonground_indices(f)
-        assert len(g_e) + len(n_e) == len(g_r) + len(n_r), f"{what}/{f}: emitted {len(g_e) + len(n_e)} vs {len(g_r) + len(n_r)}"
-        mr = np.zeros(a.shape[0], bool); mr[g_r] = True
+        assert len(g_e) + len(n_e) == emitted[f], f"{batch}/{f}: emitted {len(g_e) + len(n_e)} vs {emitted[f]}"
+        mr = masks[f]
         me = np.zeros(a.shape[0], bool); me[g_e] = True
         d = mr != me
         if d.any():
@@ -101,8 +98,7 @@ def _default_params():
     return default_params()
 
 
-@pytest.mark.skipif(not O.have_reference_build(), reason="oracle/_ref/libpwref.so was not shipped")
-def test_config3_batch_vs_reference_build():
+def test_config3_batch_vs_reference_build(refout):
     """256 frames of the benchmark's batch (config 3: synthetic KITTI-64, fresh state per frame) against the reference's own
     code on the same arrays."""
     import synth
@@ -110,32 +106,31 @@ def test_config3_batch_vs_reference_build():
     frames = [synth.make_frame(20260922, f).numpy() for f in range(nf)]
     eng = _engine(num_streams=nf)
     eng.estimate_host(frames)
-    labels, mism = _compare_with_reference(eng, frames, "config3")
+    labels, mism = _compare_with_reference(eng, frames, refout, "config3")
     print(f"parity_vs_reference: frames={nf} labels={labels} mismatches={mism}")
     assert mism <= max(4, labels // 1_000_000 * 4), f"{mism} of {labels} labels differ from the reference build"
 
 
-@pytest.mark.skipif(not O.have_reference_build(), reason="oracle/_ref/libpwref.so was not shipped")
-def test_dense_frame_vs_reference_build():
+def test_dense_frame_vs_reference_build(refout):
     """One config-5-shaped frame (~1.2 M points, patches of 20k..40k points: class X) against the reference build."""
     import synth
     a = synth.make_frame(20260922, 0, "dense1m").numpy()
     eng = _engine()
     eng.estimate_host([a])
-    labels, mism = _compare_with_reference(eng, [a], "dense")
+    labels, mism = _compare_with_reference(eng, [a], refout, "dense")
     print(f"parity_vs_reference (dense): labels={labels} mismatches={mism}")
     assert mism <= 4, f"{mism} of {labels} labels differ from the reference build"
 
 
 def test_second_device_matches_first(kitti):
     """BASELINE config 4 shards frames over the GPUs of a box: the same frames on device 1 give bit-identical lists and
-    patch records (skipped on a one-GPU box)."""
+    patch records. On a one-GPU box the second engine is an independent context on device 0: two engines that share
+    nothing must still agree bit for bit."""
     import torch
-    if torch.cuda.device_count() < 2:
-        return   # nothing to compare on a one-GPU box (not a skip: the driver's single-GPU run reports skipped tests as gaps)
     import synth
+    second = 1 if torch.cuda.device_count() > 1 else 0
     frames = [kitti[0], kitti[3], synth.make_frame(20260922, 5).numpy()]
-    e0, e1 = _engine(num_streams=3, device=0), _engine(num_streams=3, device=1)
+    e0, e1 = _engine(num_streams=3, device=0), _engine(num_streams=3, device=second)
     e0.estimate_host(frames); e1.estimate_host(frames)
     for f in range(3):
         assert np.array_equal(e0.ground_indices(f), e1.ground_indices(f)) and np.array_equal(e0.nonground_indices(f), e1.nonground_indices(f))
@@ -144,34 +139,28 @@ def test_second_device_matches_first(kitti):
     assert np.array_equal(np.sort(e1.ground_indices(0)), np.sort(orc.getGroundIndices()))
 
 
-@pytest.mark.skipif(not O.have_reference_build(), reason="oracle/_ref/libpwref_stable.so was not shipped")
-def test_index_lists_in_reference_order(kitti):
+def test_index_lists_in_reference_order(kitti, refout):
     """PWPP_ORDER_REFERENCE: ground / non-ground index LISTS identical to the reference's own code with a stable per-bin sort
     (order inside a bin: ascending z, R-VPF removals by iteration before the final rejects) — fixtures, synthetic scans, a
     wall inside a zone-0 bin (multi-iteration R-VPF) and a ~1.2 M-point frame (class-X patches sorted in global memory)."""
     import synth
-    rng = np.random.default_rng(11)
-    wall = np.r_[np.c_[4 + rng.random(6000) * 0.05, rng.random(6000) * 0.6, -1.7 + rng.random(6000) * 2.0, rng.random(6000)],
-                 np.c_[3 + rng.random(6000) * 4, rng.random(6000) * 0.6, -1.7 + rng.normal(0, 0.02, 6000), rng.random(6000)]].astype(np.float32)
-    frames = list(kitti) + [synth.make_frame(20260922, f).numpy() for f in range(6)] + [wall, synth.make_frame(20260922, 1, "dense1m").numpy()]
+    cases = [f"kitti{f}/default/fresh" for f in range(6)] + [f"synth{f}" for f in range(6)] + ["wall", "dense1"]
+    frames = list(kitti) + [synth.make_frame(20260922, f).numpy() for f in range(6)] + [wall_frame(), synth.make_frame(20260922, 1, "dense1m").numpy()]
     eng = _engine(num_streams=len(frames))
     eng.set_output_order(eng.ORDER_REFERENCE)
     eng.estimate_host(frames)
     compared = 0
-    for f, a in enumerate(frames):
-        ref = O.Reference(stable_sort=True); ref.estimate(a)
-        g_r, n_r = ref.getGroundIndices(), ref.getNongroundIndices()
-        ref.close()
+    for f, (case, a) in enumerate(zip(cases, frames)):
+        refout.check_input(case, a)
         g_e, n_e = eng.ground_indices(f), eng.nonground_indices(f)
-        if not np.array_equal(np.sort(g_r), np.sort(g_e)):
+        if not np.array_equal(digest(np.sort(g_e)), refout.digest(case, "ground_set")):
             continue   # an fp32-vs-double label flip (counted by the tests above): the lists cannot be equal then
-        assert np.array_equal(g_r, g_e), f"frame {f}: ground list order differs from the reference"
-        assert np.array_equal(n_r, n_e), f"frame {f}: non-ground list order differs from the reference"
+        assert np.array_equal(digest(g_e), refout.digest(case, "getGroundIndices")), f"{case}: ground list order differs from the reference"
+        assert np.array_equal(digest(n_e), refout.digest(case, "getNongroundIndices")), f"{case}: non-ground list order differs from the reference"
         compared += 1
     assert compared >= len(frames) - 2
     # and back: bin order (ascending index inside a bin) gives the same sets
     eng.set_output_order(eng.ORDER_BIN)
     eng.reset()
     eng.estimate_host(frames[:2])
-    ref = O.Reference(stable_sort=True); ref.estimate(frames[0])
-    assert np.array_equal(np.sort(ref.getGroundIndices()), np.sort(eng.ground_indices(0)))
+    assert np.array_equal(digest(np.sort(eng.ground_indices(0))), refout.digest("kitti0/default/fresh", "ground_set"))

@@ -1,58 +1,46 @@
 """Pins the restated oracle (oracle/pwpp_oracle.c, arith=REF32) against the reference's OWN estimateGround:
 reference cpp/patchworkpp/src/patchworkpp.cpp compiled unmodified against oracle/eigen_shim
-(oracle/_ref/libpwref_stable.so, only the per-bin sort made stable — see oracle/ref_capi.cpp).
+(oracle/_ref/libpwref_stable.so, only the per-bin sort made stable — see oracle/ref_capi.cpp), whose outputs
+tests/golden/make_golden.py recorded in tests/golden/reference_outputs.npz.
 Everything must agree BIT FOR BIT, including the emission order of the index lists."""
-import numpy as np
 import pytest
 
 import oracle_py as O
-from helpers import assert_bit_identical
+from helpers import SETS, edge_inputs
 from param_sets import PARAM_SETS
-
-pytestmark = pytest.mark.skipif(not O.have_reference_build(), reason="oracle/_ref/libpwref*.so not built")
 
 
 @pytest.mark.parametrize("pname", list(PARAM_SETS))
 @pytest.mark.parametrize("mode", ["fresh", "seq"])
-def test_fixtures_bit_identical(kitti, pname, mode):
+def test_fixtures_bit_identical(kitti, refout, pname, mode):
     mk, cols = PARAM_SETS[pname]
-    ref, orc = O.Reference(mk(), stable_sort=True), O.Oracle(mk(), O.ARITH_REF32)
+    orc = O.Oracle(mk(), O.ARITH_REF32)
     for f, a in enumerate(kitti):
         if mode == "fresh":
-            ref, orc = O.Reference(mk(), stable_sort=True), O.Oracle(mk(), O.ARITH_REF32)
-        ref.estimate(a[:, :cols]); orc.estimate(a[:, :cols])
-        assert_bit_identical(ref, orc, f"{pname}/{mode}/{f}")
+            orc = O.Oracle(mk(), O.ARITH_REF32)
+        orc.estimate(a[:, :cols])
+        refout.assert_matches(f"kitti{f}/{pname}/{mode}", a[:, :cols], orc)
 
 
-def test_synthetic_sequence_bit_identical():
+def test_synthetic_sequence_bit_identical(refout):
     import synth
-    ref, orc = O.Reference(stable_sort=True), O.Oracle(arith=O.ARITH_REF32)
+    orc = O.Oracle(arith=O.ARITH_REF32)
     for f in range(4):
         a = synth.make_frame(1234, f).numpy()
-        ref.estimate(a); orc.estimate(a)
-        assert_bit_identical(ref, orc, f"synthetic/{f}")
+        orc.estimate(a)
+        refout.assert_matches(f"synth1234_{f}/seq", a, orc)
 
 
-def test_unstable_sort_only_changes_order(kitti):
-    """The unmodified reference (std::sort) and the stable-sort variant give the same index SETS."""
+def test_unstable_sort_only_changes_order(kitti, refout):
+    """The unmodified reference (std::sort) gives the same index SETS as the stable-sort variant the oracle reproduces."""
     a = kitti[0]
-    r0, r1 = O.Reference(stable_sort=False), O.Reference(stable_sort=True)
-    r0.estimate(a); r1.estimate(a)
-    assert np.array_equal(np.sort(r0.getGroundIndices()), np.sort(r1.getGroundIndices()))
-    assert np.array_equal(np.sort(r0.getNongroundIndices()), np.sort(r1.getNongroundIndices()))
+    orc = O.Oracle(arith=O.ARITH_REF32)
+    orc.estimate(a)
+    refout.assert_matches("kitti0/default/std_sort", a, orc, SETS)
 
 
-def test_edge_inputs_bit_identical():
-    rng = np.random.default_rng(7)
-    cases = {
-        "empty": np.zeros((0, 4), np.float32),
-        "one_point": np.array([[5, 0, -1.7, 0.5]], np.float32),
-        "nine_in_one_bin": np.c_[5 + rng.random(9) * 0.1, rng.random(9) * 0.1, -1.7 + rng.random(9) * 0.01, rng.random(9)].astype(np.float32),
-        "all_out_of_range": np.c_[rng.random((50, 2)) * 1.0, rng.random((50, 2))].astype(np.float32),
-        "flat_plane": np.c_[(rng.random((5000, 2)) - 0.5) * 60, np.full(5000, -1.723), rng.random(5000)].astype(np.float32),
-        "axis_points": np.array([[10, 0, -1.7, .5], [-10, 0, -1.7, .5], [0, 10, -1.7, .5], [0, -10, -1.7, .5], [3, -0.0, -1.7, .5]] * 4, np.float32),
-    }
-    for name, a in cases.items():
-        ref, orc = O.Reference(stable_sort=True), O.Oracle(arith=O.ARITH_REF32)
-        ref.estimate(a); orc.estimate(a)
-        assert_bit_identical(ref, orc, name)
+def test_edge_inputs_bit_identical(refout):
+    for name, a in edge_inputs().items():
+        orc = O.Oracle(arith=O.ARITH_REF32)
+        orc.estimate(a)
+        refout.assert_matches(f"edge/{name}", a, orc)

@@ -1,56 +1,45 @@
 """Reference emission order (pwpp_set_output_order(PWPP_ORDER_REFERENCE), csrc/pwpp_order.cuh): the index LISTS — not just the
 sets — equal those of the reference's own code with a stable per-bin sort (oracle/_ref/libpwref_stable.so: ties in z keep
-ascending point index; with std::sort their order is unspecified in the reference itself). Kernels on the SIMT twin here,
-on the GPU in tests/test_gpu_reference.py."""
+ascending point index; with std::sort their order is unspecified in the reference itself), as recorded in
+tests/golden/reference_outputs.npz. Kernels on the SIMT twin here, on the GPU in tests/test_gpu_reference.py."""
 import numpy as np
 import pytest
 
-import oracle_py as O
-from helpers import SimtTwin
+from helpers import FLAT_PATCH_SIZES, SimtTwin, digest, flat_patch_frames, ties_frame, wall_frame
 from param_sets import PARAM_SETS
 
-pytestmark = pytest.mark.skipif(not O.have_reference_build(), reason="needs oracle/_ref/libpwref_stable.so")
-
-
-def _lists_equal(ref, tw, what):
-    for name in ("getGroundIndices", "getNongroundIndices"):
-        a, b = getattr(ref, name)(), getattr(tw, name)()
-        assert a.shape == b.shape and np.array_equal(a, b), f"{what}: {name} differs (first at {np.nonzero(a[:len(b)] != b[:len(a)])[0][:3]})"
+LISTS = ("getGroundIndices", "getNongroundIndices")
 
 
 @pytest.mark.parametrize("patch", [0, 1])
-def test_fixture_lists_in_reference_order(kitti, patch):
+def test_fixture_lists_in_reference_order(kitti, refout, patch):
     for f in (0, 3):
-        ref, tw = O.Reference(stable_sort=True), SimtTwin(order=1, patch=patch)
-        ref.estimate(kitti[f]); tw.estimate(kitti[f])
-        _lists_equal(ref, tw, f"fixture {f}")
+        tw = SimtTwin(order=1, patch=patch)
+        tw.estimate(kitti[f])
+        refout.assert_matches(f"kitti{f}/default/fresh", kitti[f], tw, LISTS)
 
 
-def test_rvpf_removals_come_first_in_iteration_order():
+def test_rvpf_removals_come_first_in_iteration_order(refout):
     """A wall inside a zone-0 bin: R-VPF removes points in several iterations; the reference appends them to the non-ground
     list iteration by iteration, each in ascending z, before the final rejects (patchworkpp.cpp:495-504, :529-541)."""
-    rng = np.random.default_rng(11)
-    wall = np.r_[np.c_[4 + rng.random(6000) * 0.05, rng.random(6000) * 0.6, -1.7 + rng.random(6000) * 2.0, rng.random(6000)],
-                 np.c_[3 + rng.random(6000) * 4, rng.random(6000) * 0.6, -1.7 + rng.normal(0, 0.02, 6000), rng.random(6000)]].astype(np.float32)
+    wall = wall_frame()
     for patch in (0, 1):
-        ref, tw = O.Reference(stable_sort=True), SimtTwin(order=1, patch=patch)
-        ref.estimate(wall); tw.estimate(wall)
-        _lists_equal(ref, tw, f"wall/patch={patch}")
+        tw = SimtTwin(order=1, patch=patch)
+        tw.estimate(wall)
+        refout.assert_matches("wall", wall, tw, LISTS)
 
 
-def test_other_parameter_set_and_synthetic_and_ties():
-    import synth
+def test_other_parameter_set_and_synthetic_and_ties(refout):
     mk, cols = PARAM_SETS["no_rvpf_tgr"]
     a = np.ascontiguousarray(conftest_kitti(1)[:, :cols])
-    ref, tw = O.Reference(mk(), stable_sort=True), SimtTwin(mk(), order=1)
-    ref.estimate(a); tw.estimate(a)
-    _lists_equal(ref, tw, "no_rvpf_tgr")
-    b = synth.make_frame(20260922, 1).numpy()
-    b[:, 2] = np.round(b[:, 2] / 0.01) * 0.01   # centimetre-quantised z: thousands of exact ties per bin
-    ref, tw = O.Reference(stable_sort=True), SimtTwin(order=1)
-    ref.estimate(b); tw.estimate(b)
-    if np.array_equal(np.sort(ref.getGroundIndices()), np.sort(tw.getGroundIndices())):   # (lattice data can flip labels between fp32 and double, DESIGN.md section 3)
-        _lists_equal(ref, tw, "ties")
+    tw = SimtTwin(mk(), order=1)
+    tw.estimate(a)
+    refout.assert_matches("kitti1/no_rvpf_tgr/fresh", a, tw, LISTS)
+    b = ties_frame()
+    tw = SimtTwin(order=1)
+    tw.estimate(b)
+    if np.array_equal(digest(np.sort(tw.getGroundIndices())), refout.digest("ties", "ground_set")):   # (lattice data can flip labels between fp32 and double, DESIGN.md section 3)
+        refout.assert_matches("ties", b, tw, LISTS)
 
 
 def conftest_kitti(f):
@@ -58,16 +47,12 @@ def conftest_kitti(f):
     return conftest.load_kitti(f)
 
 
-def test_sort_kernels_at_their_size_limits():
+def test_sort_kernels_at_their_size_limits(refout):
     """Patches whose sizes sit on the limits of the sort kernels (k_order_warp: 16-key lanes, 512-key warps; k_order_cta<128/256/512>:
     2048 / 4096 / 8192 keys) and of their padding (powers of two +- 1): one flat patch per frame, all frames in one batched call."""
-    rng = np.random.default_rng(5)
-    sizes = [10, 15, 16, 17, 31, 33, 63, 64, 65, 127, 129, 255, 256, 257, 511, 512, 513, 1023, 1025, 2047, 2048, 2049, 4095, 4096, 4097, 8191, 8192]
-    frames = [np.c_[5 + rng.random(n) * 0.5, rng.random(n) * 0.5, -1.7 + rng.normal(0, 0.03, n), rng.random(n)].astype(np.float32) for n in sizes]
+    frames = flat_patch_frames()
     tw = SimtTwin(num_streams=len(frames), order=1)
     tw.estimate_multi(frames)
-    for f, (n, a) in enumerate(zip(sizes, frames)):
-        ref = O.Reference(stable_sort=True)
-        ref.estimate(a)
+    for f, (n, a) in enumerate(zip(FLAT_PATCH_SIZES, frames)):
         tw.select(f)
-        _lists_equal(ref, tw, f"size {n}")
+        refout.assert_matches(f"flat{n}", a, tw, LISTS)

@@ -9,10 +9,11 @@ bash tools/gpu_check.sh 2>&1 | tee gpurun_out/check.log
 bash tools/gpu_profile.sh 2>&1 | tee gpurun_out/profile.log | tail -40
 cat > /tmp/one_frame.py <<'PY'
 import os, sys
-REPO = os.environ.get("GRAFT_REPO_ROOT", "/root/repo")
-sys.path[:0] = [os.path.join(REPO, "patchwork-plusplus_b200")]
-import numpy as np, pwpp_b200
-a = np.ascontiguousarray(np.load(os.path.join(REPO, "tests", "golden", "kitti_000000.npz"))["xyzi_t"].T)
+REPO = os.getcwd()   # the repository root (cd above)
+sys.path[:0] = [os.path.join(REPO, "patchwork-plusplus_b200"), os.path.join(REPO, "tests")]
+import pwpp_b200
+from conftest import load_kitti
+a = load_kitti(0)
 eng = pwpp_b200.Engine(device=0, num_streams=1); eng.set_output_order(1)
 for _ in range(6):
     eng.estimate_host([a])

@@ -1,10 +1,10 @@
 """Diagnostic: where a single-frame call spends its time (per-kernel CUDA-event times, then the un-profiled call)."""
 import os, sys, time
 REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-sys.path[:0] = [os.path.join(REPO, "patchwork-plusplus_b200")]
-import numpy as np
+sys.path[:0] = [os.path.join(REPO, "patchwork-plusplus_b200"), os.path.join(REPO, "tests")]
 import pwpp_b200
-a = np.ascontiguousarray(np.load(os.path.join(REPO, "tests", "golden", "kitti_000000.npz"))["xyzi_t"].T)
+from conftest import load_kitti
+a = load_kitti(0)
 for order in (0, 1):
     eng = pwpp_b200.Engine(device=0, num_streams=1)
     eng.set_output_order(order)
